@@ -72,7 +72,12 @@ def parse():
     ap.add_argument("--dp-transport", default="auto", choices=["auto", "nvls", "p2p"],
                     help="peer-memory DP: reduce / broadcast inside the NVSwitch (multimem) or by peer loads / stores")
     ap.add_argument("--torch-profile", default="", help="write a torch.profiler kernel table of one step to this file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step of the headline computed to DIR/<name>.npy (float32 / float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def load_workload():
@@ -158,7 +163,9 @@ class OccupancyUpdate:
         self.step += 1
 
 
-def train_step(impl, field, est, opt, scaler, batch, cfg, rk, reducer=None, sched=None, occ=None, device_counts=False):
+def train_step(impl, field, est, opt, scaler, batch, cfg, rk, reducer=None, sched=None, occ=None, device_counts=False,
+               keep=None):
+    """`keep`: a dict that receives this step's rendered rays and loss (for --dump-outputs)."""
     if occ is not None:
         occ()
     rays = impl.Rays(batch["origins"], batch["viewdirs"])
@@ -166,6 +173,8 @@ def train_step(impl, field, est, opt, scaler, batch, cfg, rk, reducer=None, sche
     rgb, acc, depth, n_samples, extra = impl.render_image(field, est, rays, render_bkgd=batch["color_bkgd"],
                                                           timestamps=batch["timestamps"], jitter=batch["jitter"], **rk,
                                                           **extra_kw)
+    if keep is not None:
+        keep.update(rgb=rgb, acc=acc, depth=depth, n_samples=n_samples)
     if not torch.is_tensor(n_samples) and n_samples == 0:
         return None, 0
     if hasattr(impl, "losses"):  # this repo: the same loss as one fused forward / backward launch
@@ -174,6 +183,8 @@ def train_step(impl, field, est, opt, scaler, batch, cfg, rk, reducer=None, sche
                                          distortion_loss=cfg.name.startswith("hypernerf"))   # run_hyper.sh: -d
     else:
         loss = torch.nn.functional.mse_loss(rgb, batch["pixels"]) + aux_losses(rgb, acc, batch["pixels"], extra, cfg.flags)
+    if keep is not None:
+        keep["loss"] = loss
     opt.zero_grad()
     if scaler is not None:
         scaler.scale(loss).backward()
@@ -385,6 +396,40 @@ class Dist:
         torch.cuda.synchronize()
 
 
+PARAM_SAMPLE = 2 ** 20        # --dump-outputs: entries kept of a larger parameter tensor
+DUMP_LIMIT = 64 * 2 ** 20     # --dump-outputs: bytes in all
+
+
+def host_outputs(keep, field=None):
+    """--dump-outputs: the tensors a caller received from the last timed step, as float32 / float64 host arrays.  A train
+    step also hands back the updated parameters: each whole, or its entries at a fixed seeded sample of PARAM_SAMPLE
+    positions."""
+    out = {}
+    for k, v in keep.items():
+        v = torch.as_tensor(v).detach()
+        out[k] = (v.float() if v.is_floating_point() else v.double()).cpu().numpy()
+    for k, p in (field.named_parameters() if field is not None else ()):
+        v = p.detach().flatten()
+        if v.numel() == 0:   # parameter-free modules (the spherical-harmonics direction encoding) have nothing to compare
+            continue
+        if v.numel() > PARAM_SAMPLE:
+            idx = torch.randint(v.numel(), (PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            v = v[idx.to(v.device)]
+        out["param." + k] = v.float().cpu().numpy()
+    return out
+
+
+def write_outputs(dirname, arrays):
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------------------
 # train-step leg
 # --------------------------------------------------------------------------------------------------------------
@@ -442,9 +487,11 @@ def train_leg(D, cb, workload, cfg, args, n_rays, steps, warmup, full: bool):
                 reducer.wait()
             opt.zero_grad()
 
+    keep = {} if (args.dump_outputs and full) else None   # the tensors of the latest resident step, for --dump-outputs
+
     def step_resident(i):
         return train_step(cb, field, est, opt, scaler, resident[i % n_host], cfg, rk, reducer, state.sched, occ,
-                          not args.host_counts)
+                          not args.host_counts, keep)
 
     # End-to-end leg: every step's inputs come from pinned host memory and every step's loss goes back to the host, both
     # inside the timed region - pipelined the way a data loader and a logger are: batch i + 1 is copied on a side stream
@@ -539,6 +586,9 @@ def train_leg(D, cb, workload, cfg, args, n_rays, steps, warmup, full: bool):
     out = {"ms": ms, "samples": dp.sum_over_ranks(samples, dev), "launches": int(launches), "occ_updates": occ.updates,
            "dp_mode": dp_mode, "rays": n_rays * world, "dropped": int(est.dropped_samples), "clocks": clocks.stop() if clocks else None,
            "h2d": sum(v.numel() * v.element_size() for v in host[0].values())}
+    if keep is not None:   # before the legs below run more steps on the same field
+        out["outputs"] = host_outputs(keep, field)
+        keep = None
     if full:
         out["ms_e2e"] = timed(step_e2e, steps)[0]
     if args.profile_steps > 0 and full:
@@ -581,8 +631,9 @@ def train_leg(D, cb, workload, cfg, args, n_rays, steps, warmup, full: bool):
 # --------------------------------------------------------------------------------------------------------------
 # render leg: full frames through render_image_test, frames interleaved over the ranks, no collective
 # --------------------------------------------------------------------------------------------------------------
-def render_leg(D, cb, workload, cfg, args, poses, times, opengl, bkgd, profile: bool):
-    """poses [F,3,4], times [F]: the whole job; rank r renders frames r, r+W, ... (strong scaling)."""
+def render_leg(D, cb, workload, cfg, args, poses, times, opengl, bkgd, profile: bool, dump: bool = False):
+    """poses [F,3,4], times [F]: the whole job; rank r renders frames r, r+W, ... (strong scaling).  `dump`: return the
+    last frame of the timed job under "outputs"."""
     from cednerf_b200 import _lib, dp
 
     dev, world, rank = D.dev, D.world, D.rank
@@ -600,10 +651,13 @@ def render_leg(D, cb, workload, cfg, args, poses, times, opengl, bkgd, profile: 
     copies = []
 
     n_samples_box = [0]
+    keep = {} if dump else None
 
     def to_host(k, res):   # 8-bit frame -> pinned ring; the copy of frame k overlaps the rendering of the next frames
         rgb, _, _, n_s = res
         n_samples_box[0] += n_s
+        if keep is not None and k == len(frames) - 1:   # frames complete out of order: keep the job's last frame
+            keep.update(rgb=rgb, acc=res[1], depth=res[2], n_samples=n_s)
         if len(copies) >= len(ring):
             copies.pop(0).synchronize()
         ring[k % len(ring)].copy_((rgb.clamp(0.0, 1.0) * 255.0).to(torch.uint8), non_blocking=True)
@@ -643,6 +697,8 @@ def render_leg(D, cb, workload, cfg, args, poses, times, opengl, bkgd, profile: 
            "samples_per_ray": round(n_all / rays, 3), "launches_per_frame": (_lib.launch_count() - l0) // max(len(mine), 1),
            # fused render per sample: 512 B table + ~50 B (SURVEY.md 8d) against the HBM copy peak, whole job
            "pipeline_frac": round(n_all * 562 / (ms * 1e-3) / 1e9 / (hbm_peak * world), 4)}
+    if keep:
+        out["outputs"] = host_outputs(keep)
     if profile and rank == 0 and frames:
         with Instrument(cb, _lib) as ins:
             cb.render_image_test(1024, field, est, cb.utils.generate_rays(K, frames[0][0], cfg.width, cfg.height, opengl),
@@ -720,9 +776,10 @@ def run_ours(args):
         return render_leg(D, cb, workload, workload.DYNERF, args, poses[idx], [k / 300.0 for k in idx], False,
                           (0.0, 0.0, 0.0), profile)
 
-    def dnerf_leg(n_frames, profile):
+    def dnerf_leg(n_frames, profile, dump=False):
         poses = torch.stack([workload.orbit_pose(4.0, 2 * 3.14159265 * k / n_frames) for k in range(n_frames)])
-        return render_leg(D, cb, workload, workload.DNERF, args, poses, [0.5] * n_frames, True, (1.0, 1.0, 1.0), profile)
+        return render_leg(D, cb, workload, workload.DNERF, args, poses, [0.5] * n_frames, True, (1.0, 1.0, 1.0), profile,
+                          dump)
 
     line = {"higher_is_better": True, "vs_baseline": None, "data": "synthetic", "n_gpus": world,
             "dtype": "f16 (MLP, tables) / f32 (marching, compositing, grads)"}
@@ -730,7 +787,8 @@ def run_ours(args):
     if args.config == "dnerf":   # configs[0]: one "step" = one 800x800 frame
         n_frames = max(args.steps, 1) * world
         for _ in range(1):
-            r = dnerf_leg(n_frames, args.profile_steps > 0)
+            r = dnerf_leg(n_frames, args.profile_steps > 0, bool(args.dump_outputs))
+        outputs = r.pop("outputs", None)
         line.update({"metric": "render_rays_per_s", "value": r["rays_per_s"], "unit": "rays/s", "steps": args.steps,
                      "warmup": 2, "ms_per_step": r["ms_per_frame_per_gpu"], "scaling": "weak",
                      "config": {"workload": r["workload"], "samples_per_ray": r["samples_per_ray"],
@@ -743,6 +801,7 @@ def run_ours(args):
         extra["render_breakdown"] = r.get("breakdown_ms_per_frame")
     else:
         t = train_leg(D, cb, workload, cfg, args, args.rays, args.steps, args.warmup, True)
+        outputs = t.pop("outputs", None)
         rays_all = t["rays"]
         line.update({
             "metric": "train_step_rays_per_s", "value": round(rays_all / (t["ms"] * 1e-3), 1), "unit": "rays/s",
@@ -809,6 +868,8 @@ def run_ours(args):
             "encoder4d_fwd_bwd_frac": [(cfgs_.get("encoder4d") or {}).get("fwd_frac"), (cfgs_.get("encoder4d") or {}).get("bwd_frac")]}
     except Exception:  # noqa: BLE001 - a summary must never cost the line
         pass
+    if rank == 0 and outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:

@@ -1,14 +1,14 @@
 """Generate tests/golden/reference_path.pt by running the REFERENCE'S OWN in-tree Python.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
+Needs a checkout of the reference (Ced-NeRF); the tests only read the file this writes:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 The reference cannot be imported as-is: cednerf/model.py exits without tinycudann, cednerf/utils.py
 and cednerf/render.py import nerfacc, cednerf/taichi_kernel/* import taichi (SURVEY.md §8c).  Those
 three absent third-party packages are replaced in sys.modules by the oracle's restatements
 (oracle.tcnn_ref / oracle.nerfacc_ref) and an inert taichi stub; everything else that executes is the
-reference's own code, unmodified, read from /root/reference:
+reference's own code, unmodified, read from the checkout:
 
     cednerf/encoder.py   SinusoidalEncoder, SinusoidalEncoderWithExp
     cednerf/utils.py     trunc_exp, render_image, render_image_test
@@ -16,6 +16,7 @@ reference's own code, unmodified, read from /root/reference:
     cednerf/model.py     DNGPradianceField
 
 The frozen vectors pin (a) oracle.cednerf_ref and (b) cednerf_b200's mirror of the same surface.
+`compact` says what of them the file keeps.
 """
 import os
 import sys
@@ -25,9 +26,7 @@ from unittest.mock import MagicMock
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = "/root/reference"
 sys.path.insert(0, REPO)
-sys.path.insert(0, REF)
 
 from oracle import nerfacc_ref as nf  # noqa: E402
 from oracle import tcnn_ref as tc  # noqa: E402
@@ -82,7 +81,34 @@ def boost_density(field):
         field.mlp_base.params.mul_(3.0)
 
 
-def main():
+HASH_GRAD_SAMPLE = 4096
+
+
+def compact(out):
+    """What reference_path.pt keeps of `out`, so that it stays under 1 MB:
+    - the four tiny-cuda-nn parameter tables of each field's initial state are not stored.  The reference draws them
+      with tcnn's default seed and boost_density scales them; tests/conftest.py repeats that and checks the result
+      against the float64 sums stored as `<set>.state_sum.<key>`.  `<set>.field_kwargs` holds the field's arguments.
+    - each hash-grid gradient keeps the entries at one fixed, seeded sample of HASH_GRAD_SAMPLE positions
+      (`grad_sample_index`) and the float64 L2 norm of the whole tensor.
+    Everything else is stored as computed."""
+    out = dict(out)
+    n_table = out["plain.field.grad.hash_encoder.params"].numel()
+    idx = torch.randperm(n_table, generator=torch.Generator().manual_seed(0))[:HASH_GRAD_SAMPLE].sort().values
+    out["grad_sample_index"] = idx.int()
+    for name, flags in FLAG_SETS.items():
+        out[f"{name}.field_kwargs"] = dict(FIELD_KW, **flags)
+        for mod in ("xyz_wrap", "hash_encoder", "mlp_base", "mlp_head"):
+            out[f"{name}.state_sum.{mod}.params"] = out.pop(f"{name}.state.{mod}.params").double().sum()
+        for part in ("field", "train"):
+            key = f"{name}.{part}.grad.hash_encoder.params"
+            g = out.pop(key)
+            out[key + ".sample"], out[key + ".norm"] = g[idx].clone(), g.double().norm()
+    return out
+
+
+def main(ref):
+    sys.path.insert(0, ref)
     install_stubs()
     from cednerf.encoder import SinusoidalEncoder, SinusoidalEncoderWithExp
     from cednerf.model import DNGPradianceField
@@ -181,9 +207,10 @@ def main():
                 "rend.gc": gc, "rend.go": go, "rend.gd": gd, "rend.gsigma": sig.grad, "rend.grgb": col.grad})
 
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_path.pt")
+    out = compact(out)
     torch.save({k: (v.clone() if torch.is_tensor(v) else v) for k, v in out.items()}, path)
-    print("wrote", path, f"{os.path.getsize(path) / 1e6:.2f} MB,", len(out), "tensors")
+    print("wrote", path, f"{os.path.getsize(path) / 1e6:.2f} MB,", len(out), "entries")
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -64,10 +64,8 @@ def test_field_against_golden(cb, golden, name):
     mv = golden[f"{name}.field.move"]
     torch.testing.assert_close(res["interal_output"]["move"].detach().cpu(), mv, rtol=2e-3, atol=2e-3 * float(mv.abs().max()))
     ((rgb * to("grgb")).sum() + (res["density"] * to("gsig")).sum()).backward()
-    for k, p in field.named_parameters():
-        key = f"{name}.field.grad.{k}"
-        if key in golden:
-            assert rel(p.grad.cpu(), golden[key]) < 1e-3, (k, rel(p.grad.cpu(), golden[key]))
+    for k, got, want in golden.grads(f"{name}.field", field):
+        assert rel(got.cpu(), want) < 1e-3, (k, rel(got.cpu(), want))
 
 
 @pytest.mark.parametrize("name", list(FLAG_SETS))
@@ -99,15 +97,13 @@ def test_render_paths_against_golden(cb, golden, name):
     loss = torch.nn.functional.mse_loss(rgb, golden[f"{name}.train.pixels"].to(DEV))
     (loss * 1024.0).backward()
     assert abs(float(loss.detach()) - float(golden[f"{name}.train.loss"])) <= 1e-3 * float(golden[f"{name}.train.loss"])
-    for k, p in field.named_parameters():
-        key = f"{name}.train.grad.{k}"
-        if key in golden:
-            # Deformation net: on this 96-ray batch ONE hidden activation of its third layer sits at 3.5e-5 (an fp16
-            # subnormal); a 1-ulp fp16 difference in one of its 64 inputs (tensor-core vs CPU fp32 summation order)
-            # moves the pre-activation across zero, the ReLU mask of that unit flips, and that single element is
-            # 2.4e-3 of the gradient norm (measured; independent of the loss scale).  Every other tensor holds 1e-3.
-            tol = 5e-3 if k.startswith("xyz_wrap") else 1e-3
-            assert rel(p.grad.cpu(), golden[key]) < tol, (k, rel(p.grad.cpu(), golden[key]))
+    for k, got, want in golden.grads(f"{name}.train", field):
+        # Deformation net: on this 96-ray batch ONE hidden activation of its third layer sits at 3.5e-5 (an fp16
+        # subnormal); a 1-ulp fp16 difference in one of its 64 inputs (tensor-core vs CPU fp32 summation order)
+        # moves the pre-activation across zero, the ReLU mask of that unit flips, and that single element is
+        # 2.4e-3 of the gradient norm (measured; independent of the loss scale).  Every other tensor holds 1e-3.
+        tol = 5e-3 if k.startswith("xyz_wrap") else 1e-3
+        assert rel(got.cpu(), want) < tol, (k, rel(got.cpu(), want))
 
     field.eval(), est.eval()
     t_frame = torch.tensor([[0.5]], device=DEV)
