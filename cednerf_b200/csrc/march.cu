@@ -204,7 +204,8 @@ __global__ void __launch_bounds__(128, MARCH_MIN_BLOCKS) march_kernel(MarchArgs 
   if (a.mask && !a.mask[oi]) {
     if (a.n_intervals) a.n_intervals[oi] = 0;
     if (a.n_samples) a.n_samples[oi] = 0;
-    if (a.termination) a.termination[r] = near;
+    // (by slot, near and termination are one array, and the fill pass leaves the planes of the rays it skips as they are)
+    if (a.termination && !(FILL && a.by_slot)) a.termination[r] = near;
     if (!FILL && a.n_runs) a.n_runs[oi] = 0;
     return;
   }
@@ -397,7 +398,11 @@ __global__ void __launch_bounds__(128, MARCH_MIN_BLOCKS) march_kernel(MarchArgs 
   }
   if (a.n_intervals) a.n_intervals[oi] = n_iv;
   if (a.n_samples) a.n_samples[oi] = n_sm;
-  if (a.termination && !(FILL && a.by_slot)) a.termination[r] = t_last;
+  // By slot (cednerf_march_round) near and termination are one array.  A ray over the run limit is marched a second time
+  // by the full-march fill, which must start from the same plane: the count pass leaves that plane in place, and the fill
+  // pass writes the termination plane instead (the same fp32 operations from the same start, so the same value).
+  const bool refilled = a.by_slot && !FILL && runs > a.run_cap;
+  if (a.termination && !refilled) a.termination[r] = t_last;
 }
 
 // Fill pass from recorded runs: no grid traversal, just the step recurrence t <- t + clamp(t*cone, step, 1e10) replayed
@@ -647,8 +652,9 @@ CEDNERF_EXPORT int cednerf_sort_boundaries(const float* t_mins, const float* t_m
   return cednerf_check_launch("cednerf_sort_boundaries");
 }
 
+// bits holds ceil(n_cells / 32) words; the unused high bits of the last one are zero
 CEDNERF_EXPORT int cednerf_occ_pack_bits(const uint8_t* binaries, int64_t n_cells, uint32_t* bits, void* stream) {
-  CEDNERF_REQUIRE(n_cells > 0 && (n_cells % 32) == 0, "cell count must be a multiple of 32");
+  CEDNERF_REQUIRE(n_cells > 0, "empty grid");
   pack_bits_kernel<<<cednerf_blocks(n_cells, 256), 256, 0, (cudaStream_t)stream>>>(binaries, n_cells, bits);
   return cednerf_check_launch("cednerf_occ_pack_bits");
 }
@@ -1013,9 +1019,12 @@ CEDNERF_EXPORT int cednerf_render_round_begin(int32_t* state, int64_t n_rays, in
 }
 
 // One marching pass of a round over the alive list (first state[0] entries of `alive`; n_bound >= state[0] sizes the
-// launch).  near_term [n_rays]: the rays' start planes on entry; the count pass (fill == 0) leaves the termination
-// planes there.  Per-slot outputs: n_samples, runs.  fill == 1: the full-march fill for the slots flagged in slot_mask
-// (rays over the run limit), at offsets[slot].  The sample limit k is read from state[1].
+// launch).  near_term [n_rays]: the rays' start planes on entry, their termination planes once both passes have run: the
+// count pass (fill == 0) writes them for the rays within the run limit, the fill pass for the rays over it (it marches
+// those again from their start planes).  Per-slot outputs: n_samples, runs.  fill == 1: the full-march fill for the slots
+// flagged in slot_mask (rays over the run limit), at offsets[slot].  It writes a ray's whole count, so the packed
+// buffers must hold every sample of the round: the rounds of render_image_test allocate n_rays * max(1, min_samples) >=
+// n_alive * k (utils._render_rounds_gen) and never truncate.  The sample limit k is read from state[1].
 CEDNERF_EXPORT int cednerf_march_round(int fill, const float* rays_o, const float* rays_d, int64_t n_bound,
                                        const uint32_t* occ_bits, const float* aabbs, int n_levels, int resolution,
                                        float* near_term, float far_const, float step_size, float cone_angle,
@@ -1038,7 +1047,7 @@ CEDNERF_EXPORT int cednerf_march_round(int fill, const float* rays_o, const floa
   a.step_size = step_size, a.cone_angle = cone_angle, a.limit = 0, a.mask = fill ? slot_mask : nullptr;
   a.t_sorted = t_sorted, a.t_indices = t_indices, a.hits = hits;
   a.sm_starts = offsets, a.t_starts = t_starts, a.t_ends = t_ends, a.ray_indices = ray_indices;
-  a.n_samples = fill ? nullptr : n_samples, a.termination = fill ? nullptr : near_term;
+  a.n_samples = fill ? nullptr : n_samples, a.termination = near_term;
   a.run_t = fill ? nullptr : run_t, a.run_n = fill ? nullptr : run_n, a.n_runs = fill ? nullptr : n_runs, a.run_cap = run_cap;
   a.order = alive, a.n_active_dev = state, a.limit_dev = state + 1, a.by_slot = 1;
   a.coarse = (resolution % 4 == 0) ? occ_coarse : nullptr;

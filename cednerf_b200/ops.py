@@ -48,13 +48,13 @@ def sort_boundaries(t_mins, t_maxs):
 
 
 def pack_occupancy(binaries: torch.Tensor) -> torch.Tensor:
-    """bool [L,R,R,R] -> uint32 bit field (int32 storage), 1 bit per cell in the same order."""
+    """bool [L,R,R,R] -> uint32 bit field (int32 storage), 1 bit per cell in the same order, the last word zero-padded."""
     _lib.check_device()
     b = binaries.detach().contiguous()
     if b.dtype != torch.bool and b.dtype != U8:
         b = b.to(torch.bool)
     n_cells = b.numel()
-    bits = torch.empty(n_cells // 32, dtype=I32, device=b.device)
+    bits = torch.empty((n_cells + 31) // 32, dtype=I32, device=b.device)
     call("cednerf_occ_pack_bits", ptr(b), n_cells, ptr(bits), stream())
     return bits
 

@@ -340,6 +340,15 @@ def render_images_test(max_samples, radiance_field, estimator, rays_list, timest
     n_frames = len(rays_list)
     results = [None] * n_frames
     main = torch.cuda.current_stream()
+    # The frames share caches derived from the occupancy grid and the parameters.  Build them here, on the calling
+    # stream, which every frame stream waits for: built inside the first frame's stream, they would be read by the
+    # other frames' streams with nothing ordering the reads after the writes.
+    bits = nerfacc.grid.occupancy_bits(estimator.binaries)
+    ops.occupancy_coarse(bits, int(estimator.aabbs.shape[0]), int(estimator.binaries.shape[1]))
+    if getattr(radiance_field, "fused_supported", lambda: False)():
+        radiance_field.hash_encoder.table_f16()
+        for net in (radiance_field.xyz_wrap.network, radiance_field.mlp_base, radiance_field.mlp_head):
+            net.weight_image()
     streams = _frame_streams(max(1, min(int(concurrency), n_frames)))
     free, active, nxt = list(streams), [], 0
     while active or nxt < n_frames:

@@ -46,7 +46,7 @@ int cednerf_ray_aabb_intersect(const float* rays_o, const float* rays_d, int64_t
 int cednerf_sort_boundaries(const float* t_mins, const float* t_maxs, int64_t n_rays, int n_levels, float* t_sorted,
                             int64_t* t_indices, void* stream);
 /* OccGridEstimator.binaries (bool bytes [L,R,R,R]) -> 1 bit per cell, same cell order */
-int cednerf_occ_pack_bits(const uint8_t* binaries, int64_t n_cells, uint32_t* bits, void* stream);
+int cednerf_occ_pack_bits(const uint8_t* binaries, int64_t n_cells, uint32_t* bits /*ceil(n_cells / 32) words*/, void* stream);
 /* binaries = occs > *threshold_dev, plus the bit field (last line of OccGridEstimator._update; train_real.py:332-336) */
 int cednerf_occ_threshold_pack(const float* occs, int64_t n_cells, const float* threshold_dev, uint8_t* binaries,
                                uint32_t* bits, void* stream);
@@ -277,7 +277,7 @@ int cednerf_render_round_begin(int32_t* state, int64_t n_rays, int max_samples, 
                                const int64_t* prev_totals /*nullable*/, int64_t* total /*nullable, += prev_totals[0]*/,
                                void* stream);
 int cednerf_march_round(int fill, const float* rays_o, const float* rays_d, int64_t n_bound, const uint32_t* occ_bits,
-                        const float* aabbs, int n_levels, int resolution, float* near_term /*[n_rays] in: start planes. out (count pass): termination planes*/, float far_const, float step_size, float cone_angle,
+                        const float* aabbs, int n_levels, int resolution, float* near_term /*[n_rays] in: start planes. out (count pass, then fill pass for the rays over the run limit): termination planes*/, float far_const, float step_size, float cone_angle,
                         const float* t_sorted, const int64_t* t_indices, const uint8_t* hits, const int32_t* alive,
                         const int32_t* state, const uint8_t* slot_mask /*fill*/, const int64_t* offsets /*fill*/,
                         float* t_starts, float* t_ends, int64_t* ray_indices, int32_t* n_samples /*count, per slot*/,

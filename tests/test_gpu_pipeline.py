@@ -332,16 +332,22 @@ def test_device_count_sampling_matches_the_host_count_path(cb):
     assert int(short[3]) < n and est.dropped_samples > 0
 
 
-def test_device_resident_render_rounds_match_the_host_driven_loop(cb):
+def test_device_resident_render_rounds_match_the_host_driven_loop(cb, monkeypatch):
     """render_image_test with the alive list / per-round k / termination test on the device against the loop that reads
     `alive.sum()` back every round (cednerf/utils.py:231): same image, same sample total - per ray the two paths do the
-    same arithmetic on the same samples, only the packing order of the rays inside a round differs."""
-    from cednerf_b200 import utils as U, workload as w
+    same arithmetic on the same samples, only the packing order of the rays inside a round differs.  The last input is a
+    checkerboard occupancy with a run limit of 1: every ray with more than one run takes the full-march fallback fill."""
+    from cednerf_b200 import ops, utils as U, workload as w
 
-    for cfg, opengl in ((w.TINY, False), (w.DNERF, True)):
+    for cfg, opengl, checker in ((w.TINY, False, False), (w.DNERF, True, False), (w.TINY, False, True)):
         rk = w.render_kwargs(cfg)
         est, field = w.build_scene(cfg, DEV, cb, seed=42)
         est.eval(), field.eval()
+        if checker:
+            i = torch.arange(cfg.occ_res, device=DEV)
+            cells = ((i[:, None, None] + i[None, :, None] + i[None, None, :]) % 2) == 0
+            est.binaries = cells[None].expand_as(est.binaries).contiguous()
+            monkeypatch.setattr(ops.MarchInputs, "RUN_CAP", 1)
         pose = w.orbit_pose(4.0, 0.3) if opengl else w.spiral_poses(cfg, 8)[3]
         o, d = w.pose_rays(cfg, pose, opengl, DEV)
         if cfg is w.DNERF:   # a 96 x 128 window of the 800 x 800 frame
