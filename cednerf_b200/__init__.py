@@ -11,16 +11,18 @@ Module map (reference surface -> here):
     apex FusedAdam + torch GradScaler      cednerf_b200.optim
     loss of train_real.py:369-409          cednerf_b200.losses
     datasets/dnerf_3d_video_IS.py (per-step importance sampling)   cednerf_b200.importance
+    pytorch_msssim.ms_ssim (evaluation, train_real.py:497-499)     cednerf_b200.metrics
 All compute goes through libcednerf_b200.so (include/cednerf_b200.h); there is no CPU fallback."""
 from . import _lib
 
 _lib.load()  # fail loudly if the CUDA library has not been built
 
-from . import encoder, hash_encoder, importance, losses, model, nerfacc, ops, optim, render, tcnn, utils  # noqa: E402
+from . import encoder, hash_encoder, importance, losses, metrics, model, nerfacc, ops, optim, render, tcnn, utils  # noqa: E402
 from .model import DNGPradianceField  # noqa: E402
 from .nerfacc import OccGridEstimator  # noqa: E402
 from .render import rendering  # noqa: E402
 from .utils import Rays, render_image, render_image_test, render_images_test  # noqa: E402
 
 __all__ = ["DNGPradianceField", "OccGridEstimator", "rendering", "render_image", "render_image_test", "render_images_test", "Rays",
-           "nerfacc", "tcnn", "hash_encoder", "encoder", "model", "render", "utils", "ops", "optim", "losses", "importance"]
+           "nerfacc", "tcnn", "hash_encoder", "encoder", "model", "render", "utils", "ops", "optim", "losses", "importance",
+           "metrics"]

@@ -154,6 +154,7 @@ _SIGNATURES = {
     "cednerf_dp_found_inf": "Pppp",
     "cednerf_dp_adam": "Dpppfffip",
     "cednerf_dp_adam_small": "Spppfffip",
+    "cednerf_ms_ssim": "ppppllllpffppp",
 }
 _CT = {"p": ctypes.c_void_p, "i": ctypes.c_int, "l": ctypes.c_int64, "f": ctypes.c_float,
        "G": ctypes.POINTER(GridLevels), "M": ctypes.POINTER(MlpDesc), "F": ctypes.POINTER(FieldDesc),
@@ -190,6 +191,8 @@ def load() -> ctypes.CDLL:
     lib.cednerf_distortion_workspace_bytes.argtypes = []
     lib.cednerf_sample_order_workspace_bytes.restype = ctypes.c_int64
     lib.cednerf_sample_order_workspace_bytes.argtypes = [ctypes.c_int64]
+    lib.cednerf_ms_ssim_workspace_bytes.restype = ctypes.c_int64
+    lib.cednerf_ms_ssim_workspace_bytes.argtypes = [ctypes.c_int64] * 4
     for name, sig in _SIGNATURES.items():
         fn = getattr(lib, name)
         fn.restype = ctypes.c_int
@@ -201,7 +204,8 @@ def load() -> ctypes.CDLL:
 def exported_symbols():
     return sorted(list(_SIGNATURES) + ["cednerf_last_error", "cednerf_abi_version", "cednerf_check_device",
                                        "cednerf_scan_workspace_bytes", "cednerf_launch_count", "cednerf_field_saved_bytes",
-                                       "cednerf_field_bwd_workspace_bytes", "cednerf_dp_ctrl_bytes", "cednerf_topk_workspace_bytes", "cednerf_sample_order_workspace_bytes", "cednerf_distortion_workspace_bytes", "cednerf_render_round_bytes"])
+                                       "cednerf_field_bwd_workspace_bytes", "cednerf_dp_ctrl_bytes", "cednerf_topk_workspace_bytes", "cednerf_sample_order_workspace_bytes", "cednerf_distortion_workspace_bytes", "cednerf_render_round_bytes",
+                                       "cednerf_ms_ssim_workspace_bytes"])
 
 
 def ptr(t: Optional[torch.Tensor]):

@@ -502,6 +502,20 @@ int cednerf_importance_batch(const int64_t* cells, int64_t k, int subsample, int
                              const float* timestamps, float* origins, float* viewdirs, float* rgb, float* timestamps_out,
                              int64_t* image_id_out, int64_t* pixel_index_out, void* stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * MS-SSIM of the evaluation after training (train_real.py:497-499 -> pytorch_msssim.ms_ssim, 4-D inputs, 11-tap window
+ * of sigma 1.5, the five default weights; restated in oracle/metrics_ref.py).  x, y: fp32 [n, c, h, w] at any element
+ * strides (x_strides_host / y_strides_host: 4 int64 each; x and y may differ), 160 < h, w <= 65536, n * c <= 65535.
+ * taps_host: the 11 fp32 Gaussian taps; c1 = (0.01 data_range)^2, c2 = (0.03 data_range)^2.  out: n + 1 floats, the
+ * value of each image (mean over channels), then the mean over all images and channels.  6 launches (one per scale, one
+ * to finish), no atomics.  work: cednerf_ms_ssim_workspace_bytes(n, c, h, w) (-1: sizes refused), laid out as: the
+ * pooled planes of scales 1..4 (x then y, fp32 [n * c, h_s, w_s], h_s = (h_{s-1} + 1) / 2), then at the next multiple
+ * of 16 bytes the per-scale means (fp64 [5][n * c][2]: ssim_map, cs_map), then the per-tile partials. */
+int64_t cednerf_ms_ssim_workspace_bytes(int64_t n, int64_t c, int64_t h, int64_t w);
+int cednerf_ms_ssim(const float* x, const int64_t* x_strides_host, const float* y, const int64_t* y_strides_host,
+                    int64_t n, int64_t c, int64_t h, int64_t w, const float* taps_host, float c1, float c2, void* work,
+                    float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
