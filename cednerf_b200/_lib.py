@@ -119,9 +119,8 @@ _SIGNATURES = {
     "cednerf_mlp_bwd": "ppppMlpippp",
     "cednerf_field_fwd": "ppppppppilppppFpppp",
     "cednerf_occ_update_level": "plpppiffpppFpppp",
-    "cednerf_field_train_fwd": "ppppppilpppppFppppppppp",
-    "cednerf_field_train_bwd": "ppppppilpppppFpppppppppppppippp",
-    "cednerf_sample_order": "ppppplpffffffppp",
+    "cednerf_field_train_fwd": "ppppppilpppppFpppppppp",
+    "cednerf_field_train_bwd": "ppppppilpppppFpppppppppppppipp",
     "cednerf_ray_offsets": "pllpp",
     "cednerf_composite_fwd": "pppppppillpppppppifp",
     "cednerf_composite_bwd": "pppppppillppppppppppfp",
@@ -189,8 +188,6 @@ def load() -> ctypes.CDLL:
         raise ImportError("cednerf_b200: CednerfRenderRound layout mismatch between the library and _lib.RenderRound")
     lib.cednerf_distortion_workspace_bytes.restype = ctypes.c_int64
     lib.cednerf_distortion_workspace_bytes.argtypes = []
-    lib.cednerf_sample_order_workspace_bytes.restype = ctypes.c_int64
-    lib.cednerf_sample_order_workspace_bytes.argtypes = [ctypes.c_int64]
     lib.cednerf_ms_ssim_workspace_bytes.restype = ctypes.c_int64
     lib.cednerf_ms_ssim_workspace_bytes.argtypes = [ctypes.c_int64] * 4
     for name, sig in _SIGNATURES.items():
@@ -204,7 +201,7 @@ def load() -> ctypes.CDLL:
 def exported_symbols():
     return sorted(list(_SIGNATURES) + ["cednerf_last_error", "cednerf_abi_version", "cednerf_check_device",
                                        "cednerf_scan_workspace_bytes", "cednerf_launch_count", "cednerf_field_saved_bytes",
-                                       "cednerf_field_bwd_workspace_bytes", "cednerf_dp_ctrl_bytes", "cednerf_topk_workspace_bytes", "cednerf_sample_order_workspace_bytes", "cednerf_distortion_workspace_bytes", "cednerf_render_round_bytes",
+                                       "cednerf_field_bwd_workspace_bytes", "cednerf_dp_ctrl_bytes", "cednerf_topk_workspace_bytes", "cednerf_distortion_workspace_bytes", "cednerf_render_round_bytes",
                                        "cednerf_ms_ssim_workspace_bytes"])
 
 

@@ -23,7 +23,7 @@ void cednerf_set_error(const char* fmt, ...) {
 
 CEDNERF_EXPORT const char* cednerf_last_error(void) { return g_last_error; }
 
-CEDNERF_EXPORT int cednerf_abi_version(void) { return 3; }
+CEDNERF_EXPORT int cednerf_abi_version(void) { return 4; }
 
 // 0 when the current device can run this library (compute capability 10.x), else a negative code.
 CEDNERF_EXPORT int cednerf_check_device(void) {

@@ -84,14 +84,8 @@ struct TrainArgs {
   float* d_params[4];
   uint32_t tmem_cols;
   int flush_tiles;  // > 0: flush the TMEM weight-gradient accumulators every this many tiles of a group
-  // nullable: walk the samples in this order (cednerf_sample_order: spatial buckets).  Kernel-internal sample index s ->
-  // entry order[s] of every EXTERNAL per-sample array (packed samples, sigma / rgb / latent / selector / move and the
-  // incoming gradients); the saved activations and the work buffers are laid out by s.
-  const int32_t* order;
   CednerfFieldDesc d;
 };
-
-__device__ __forceinline__ int64_t ext_index(const TrainArgs& a, int64_t s) { return a.order ? (int64_t)a.order[s] : s; }
 
 __device__ __forceinline__ int64_t live_count(const TrainArgs& a) {
   if (!a.n_dev) return a.n;
@@ -192,8 +186,7 @@ __global__ void __launch_bounds__(TRAIN_FWD_GROUPS * 128, 1) field_train_fwd_ker
     long long phase_t = clock64();
     if (gtid == 0) atomicAdd(&g_train_phase_clocks[11], 1ull);
 #endif
-    const int64_t e = ok ? ext_index(a, s) : 0;  // where this sample lives in the caller's arrays
-    if (ok) packed_sample(a.ridx, a.t0, a.t1, a.rays_o, a.rays_d, a.t, a.t_stride, e, x, tv, ray);
+    if (ok) packed_sample(a.ridx, a.t0, a.t1, a.rays_o, a.rays_d, a.t, a.t_stride, s, x, tv, ray);
     // ---- deformation net ---------------------------------------------------------------------------------------
     frequency_row<true>(abuf, gtid, x[0], x[1], x[2], tv);
     fence_proxy_async();
@@ -226,8 +219,8 @@ __global__ void __launch_bounds__(TRAIN_FWD_GROUPS * 128, 1) field_train_fwd_ker
     if (ok) {
       float* xs = reinterpret_cast<float*>(a.saved + sl.xn) + 3 * s;
       xs[0] = xn[0], xs[1] = xn[1], xs[2] = xn[2];
-      a.move[3 * e] = mv[0], a.move[3 * e + 1] = mv[1], a.move[3 * e + 2] = mv[2];
-      a.selector[e] = (uint8_t)selector;
+      a.move[3 * s] = mv[0], a.move[3 * s + 1] = mv[1], a.move[3 * s + 2] = mv[2];
+      a.selector[s] = (uint8_t)selector;
     }
     TPHASE_MARK(2);
     // ---- density net input: [hash 2L | time 9 | 1.0 ...] ---------------------------------------------------------
@@ -287,7 +280,7 @@ __global__ void __launch_bounds__(TRAIN_FWD_GROUPS * 128, 1) field_train_fwd_ker
         uint4* dst = reinterpret_cast<uint4*>(a.saved + sl.o2 + s * 32);
         dst[0] = make_uint4(p[0], p[1], p[2], p[3]);
         dst[1] = make_uint4(p[4], p[5], p[6], p[7]);
-        a.sigma[e] = selector ? expf(rnd16(o2[0]) - 1.f) : 0.f;
+        a.sigma[s] = selector ? expf(rnd16(o2[0]) - 1.f) : 0.f;
       }
       // ---- colour net ------------------------------------------------------------------------------------------
       float dir[3] = {0.f, 0.f, 1.f}, feat15[15];
@@ -309,7 +302,7 @@ __global__ void __launch_bounds__(TRAIN_FWD_GROUPS * 128, 1) field_train_fwd_ker
       tmem_ld_wait();
       if (ok) {
 #pragma unroll
-        for (int k = 0; k < 3; ++k) a.rgb[3 * e + k] = 1.f / (1.f + expf(-rnd16(r[k])));
+        for (int k = 0; k < 3; ++k) a.rgb[3 * s + k] = 1.f / (1.f + expf(-rnd16(r[k])));
       }
     }
     if (has4) {
@@ -338,7 +331,7 @@ __global__ void __launch_bounds__(TRAIN_FWD_GROUPS * 128, 1) field_train_fwd_ker
             const uint4* fsrc = reinterpret_cast<const uint4*>(a.saved + sl.in2 + s * k2 * 2) + 2 * cb;
             const uint4 f0 = fsrc[0], f1 = fsrc[1];
             const uint32_t fw[8] = {f0.x, f0.y, f0.z, f0.w, f1.x, f1.y, f1.z, f1.w};
-            float4* lo = reinterpret_cast<float4*>(a.latent + e * 32 + cb * 16);
+            float4* lo = reinterpret_cast<float4*>(a.latent + s * 32 + cb * 16);
             float lv[16];
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
@@ -382,14 +375,13 @@ __device__ __forceinline__ void predictor_dout(const TrainArgs& a, const SavedLa
   const int k2 = a.d.f2.dim_in[0];
   const uint4* ps = reinterpret_cast<const uint4*>(a.saved + sl.o4 + s * 64) + 2 * cb;
   const uint4* fs = reinterpret_cast<const uint4*>(a.saved + sl.in2 + s * k2 * 2) + 2 * cb;
-  const int64_t e = ext_index(a, s);
-  const bool sel = a.selector[e] != 0;
+  const bool sel = a.selector[s] != 0;
 #pragma unroll
   for (int c = 0; c < 2; ++c) {
     const uint4 p = ps[c], f = fs[c];
     const uint32_t pw[4] = {p.x, p.y, p.z, p.w}, fw[4] = {f.x, f.y, f.z, f.w};
-    const float4 l0 = *reinterpret_cast<const float4*>(a.d_latent + e * 32 + (2 * cb + c) * 8);
-    const float4 l1 = *reinterpret_cast<const float4*>(a.d_latent + e * 32 + (2 * cb + c) * 8 + 4);
+    const float4 l0 = *reinterpret_cast<const float4*>(a.d_latent + s * 32 + (2 * cb + c) * 8);
+    const float4 l1 = *reinterpret_cast<const float4*>(a.d_latent + s * 32 + (2 * cb + c) * 8 + 4);
     const float lg[8] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w};
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
@@ -417,9 +409,8 @@ __device__ __forceinline__ void make_dout(const TrainArgs& a, const SavedLayout&
       float g[3];
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
-        const int64_t e = ext_index(a, s);
-        const float c = a.rgb[3 * e + k];
-        g[k] = a.d_rgb[3 * e + k] * c * (1.f - c);  // sigmoid backward (model.py:464-465)
+        const float c = a.rgb[3 * s + k];
+        g[k] = a.d_rgb[3 * s + k] * c * (1.f - c);  // sigmoid backward (model.py:464-465)
       }
       w[0] = pack_h2(g[0], g[1]);
       w[1] = pack_h2(g[2], 0.f);
@@ -429,8 +420,7 @@ __device__ __forceinline__ void make_dout(const TrainArgs& a, const SavedLayout&
       w[0] = g0.x, w[1] = g0.y, w[2] = g0.z, w[3] = g0.w, w[4] = g1.x, w[5] = g1.y, w[6] = g1.z, w[7] = g1.w;
       const __half raw = *reinterpret_cast<const __half*>(a.saved + sl.o2 + s * 32);
       // trunc_exp backward: g * exp(clamp(raw - 1, max = 15)), times the selector (utils.py:27-43, model.py:414-417)
-      const int64_t e = ext_index(a, s);
-      const float gs = a.selector[e] ? a.d_sigma[e] * expf(fminf(__half2float(raw) - 1.f, 15.f)) : 0.f;
+      const float gs = a.selector[s] ? a.d_sigma[s] * expf(fminf(__half2float(raw) - 1.f, 15.f)) : 0.f;
       const float hi = __half2float(__ushort_as_half((unsigned short)(w[0] >> 16)));
       w[0] = pack_h2(gs, hi);
     } else if constexpr (NET == 4) {
@@ -497,7 +487,7 @@ __device__ __forceinline__ void make_input(const TrainArgs& a, const SavedLayout
   }
   float x[3], tv;
   int64_t ray;
-  packed_sample(a.ridx, a.t0, a.t1, a.rays_o, a.rays_d, a.t, a.t_stride, ext_index(a, s), x, tv, ray);
+  packed_sample(a.ridx, a.t0, a.t1, a.rays_o, a.rays_d, a.t, a.t_stride, s, x, tv, ray);
   if constexpr (NET == 1) {
     frequency_row<true>(tile, row, x[0], x[1], x[2], tv);
   } else if constexpr (NET == 4) {
@@ -899,8 +889,8 @@ CEDNERF_EXPORT int cednerf_field_train_fwd(const int64_t* ray_indices, const flo
                                            int t_stride, int64_t n, const void* image_deform, const void* image_density,
                                            const void* image_colour, const void* image_predict, const void* table_f16,
                                            const CednerfFieldDesc* desc, float* sigma, float* rgb, float* latent,
-                                           uint8_t* selector, float* move, void* saved, const int32_t* sample_order,
-                                           const int64_t* n_device, void* stream) {
+                                           uint8_t* selector, float* move, void* saved, const int64_t* n_device,
+                                           void* stream) {
   CEDNERF_REQUIRE(check_train_desc(desc), "bad field descriptor");
   CEDNERF_REQUIRE(n >= 0 && ray_indices && t_starts && t_ends && rays_o && rays_d && timestamps && sigma && rgb &&
                       selector && move && saved,
@@ -920,7 +910,7 @@ CEDNERF_EXPORT int cednerf_field_train_fwd(const int64_t* ray_indices, const flo
   a.img[2] = (const uint8_t*)image_colour, a.img[3] = (const uint8_t*)image_predict;
   a.table = (const __half*)table_f16;
   a.sigma = sigma, a.rgb = rgb, a.latent = desc->f4.n_layers > 0 ? latent : nullptr, a.selector = selector, a.move = move;
-  a.saved = (uint8_t*)saved, a.order = sample_order;
+  a.saved = (uint8_t*)saved;
   a.d = *desc;
   const int64_t tiles = (n + MLP_TILE - 1) / MLP_TILE;
   const int64_t ctas = tiles;  // tiles go round-robin over CTAs first, then over the groups of a CTA
@@ -939,8 +929,7 @@ CEDNERF_EXPORT int cednerf_field_train_bwd(const int64_t* ray_indices, const flo
                                            const uint8_t* selector, const void* saved, const float* d_sigma,
                                            const float* d_rgb, const float* d_latent, void* work, float* d_params_deform,
                                            float* d_params_density, float* d_params_colour, float* d_params_predict,
-                                           float* g_table, int phase, const int32_t* sample_order,
-                                           const int64_t* n_device, void* stream) {
+                                           float* g_table, int phase, const int64_t* n_device, void* stream) {
   CEDNERF_REQUIRE(check_train_desc(desc), "bad field descriptor");
   CEDNERF_REQUIRE(phase >= 0 && phase <= 2, "phase: 0 all, 1 up to the table gradient, 2 the rest");
   CEDNERF_REQUIRE(n >= 0 && ray_indices && t_starts && t_ends && rays_o && rays_d && timestamps && rgb && selector &&
@@ -958,7 +947,7 @@ CEDNERF_EXPORT int cednerf_field_train_bwd(const int64_t* ray_indices, const flo
   a.img[2] = (const uint8_t*)image_colour, a.img[3] = (const uint8_t*)image_predict;
   a.table = (const __half*)table_f16;
   a.sigma = const_cast<float*>(sigma), a.rgb = const_cast<float*>(rgb), a.selector = const_cast<uint8_t*>(selector);
-  a.saved = (uint8_t*)saved, a.order = sample_order;
+  a.saved = (uint8_t*)saved;
   a.d_sigma = d_sigma, a.d_rgb = d_rgb, a.d_latent = d_latent, a.work = (uint8_t*)work;
   a.d_params[0] = d_params_deform, a.d_params[1] = d_params_density, a.d_params[2] = d_params_colour;
   a.d_params[3] = d_params_predict;

@@ -115,7 +115,7 @@ class DNGPradianceField(torch.nn.Module):
         return (self.fused_supported() and not self.use_weight_predict
                 and (not self.use_feat_predict or self.hash_encoder.n_levels == 16))
 
-    def fused_train(self, ridx, t0, t1, rays_o, rays_d, timestamps, t_stride, order_box=None):
+    def fused_train(self, ridx, t0, t1, rays_o, rays_d, timestamps, t_stride):
         """Training forward of `forward(positions, t, directions)` on packed samples, differentiable w.r.t. every
         parameter: -> (rgb [n,3], {"density", "base_mlp_out", "interal_output"}) like the op-by-op path."""
         f4 = self.mlp_feat_prediction.network if self.use_feat_predict else None
@@ -125,8 +125,7 @@ class DNGPradianceField(torch.nn.Module):
             self.xyz_wrap.network.params, self.mlp_base.params, self.mlp_head.params,
             None if f4 is None else f4.params, self.hash_encoder.params.view(-1, 2), self._field_desc(), images,
             self.hash_encoder.table_f16(), ridx, t0, t1, rays_o, rays_d, timestamps, t_stride, f4 is not None,
-            None if ops.counts_of(ridx) is None else ops.counts_of(ridx)[1],
-            None if order_box is None else tuple(float(v) for v in order_box))
+            None if ops.counts_of(ridx) is None else ops.counts_of(ridx)[1])
         io = {"move": torch.linalg.norm(move, dim=-1) if (self.use_time_embedding and self.use_time_attenuation) else move}
         if self.use_feat_predict:
             io["selector"], io["latent_losses"] = selector, latent

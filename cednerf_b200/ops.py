@@ -705,13 +705,6 @@ def field_fwd(desc: FieldDesc, images, table_f16, n: int, sigma_only: bool, pack
 
 _table_grad_hook = None
 
-# FieldTrainFunction walks batches of at least this many samples in spatial-bucket order (None: never).  OFF by default:
-# measured on the DyNeRF-shaped step (profiles/r2s_sample_order.md) the walk itself is worth 0.24 ms (forward 0.63 ->
-# 0.46, backward 1.41 -> 1.35 with physically sorted arrays), but the indirection puts two more dependent loads on the
-# critical path of every tile of these latency-bound kernels (forward 0.57, backward 1.49) and the ordering costs 0.07 ms.
-SAMPLE_ORDER_MIN = None
-
-
 def set_table_grad_hook(fn):
     """fn(g_table) is called from the fused training backward as soon as the hash-table gradient is complete, before
     the encoding's dL/dx and the deformation-net backward are launched (dp.GradAllReducer starts its all-reduce there).
@@ -737,7 +730,7 @@ class FieldTrainFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, p1, p2, p3, p4, table, desc, images, table_f16, ridx, t0, t1, rays_o, rays_d, ts, t_stride,
-                want_latent, n_dev=None, order_box=None):
+                want_latent, n_dev=None):
         _lib.check_device()
         lib = _lib.load()
         n, dev = t0.numel(), t0.device
@@ -752,22 +745,9 @@ class FieldTrainFunction(torch.autograd.Function):
         # capacity in steps of 32 Ki samples: the visible-sample count changes a little every step, and a 1 GB buffer that
         # grows by a few KB would make the caching allocator cudaMalloc (and sometimes free + retry) in the hot loop
         saved = torch.empty(max(int(lib.cednerf_field_saved_bytes(ctypes.byref(desc), _sticky_capacity(n))), 16), dtype=U8, device=dev)
-        # opt-in (SAMPLE_ORDER_MIN): walk the visible samples in spatial buckets (csrc/sample_order.cu) - ~4 samples per ray
-        # from rays drawn at random leave the lanes of a warp in unrelated places, and every hash-grid gather then touches
-        # 32 different sectors; in bucket order the coarse and middle levels coalesce
-        order = None
-        if SAMPLE_ORDER_MIN is not None and n >= SAMPLE_ORDER_MIN:
-            order = _sempty(n, dtype=torch.int32, device=dev)
-            ws = torch.empty(int(lib.cednerf_sample_order_workspace_bytes(_sticky_capacity(n))), dtype=U8, device=dev)
-            # buckets over the caller's region of interest (the estimator's level-0 box) when it is known: the field's own
-            # aabb is the OUTERMOST occupancy level (8 x the region on DyNeRF), i.e. 16 buckets per axis where it matters
-            bx = [float(v) for v in (order_box if order_box is not None else desc.aabb)]
-            call("cednerf_sample_order", ptr(ridx), ptr(t0), ptr(t1), ptr(rays_o), ptr(rays_d), n, ptr(n_dev), *bx,
-                 ptr(ws), ptr(order), stream())
         call("cednerf_field_train_fwd", ptr(ridx), ptr(t0), ptr(t1), ptr(rays_o), ptr(rays_d), ptr(ts), int(t_stride), n,
              ptr(images[0]), ptr(images[1]), ptr(images[2]), ptr(images[3]), ptr(table_f16), ctypes.byref(desc),
-             ptr(sigma), ptr(rgb), ptr(latent), ptr(selector), ptr(move), ptr(saved), ptr(order), ptr(n_dev), stream())
-        ctx.order = order
+             ptr(sigma), ptr(rgb), ptr(latent), ptr(selector), ptr(move), ptr(saved), ptr(n_dev), stream())
         ctx.save_for_backward(ridx, t0, t1, rays_o, rays_d, ts, sigma, rgb, selector, saved, table_f16, images[0],
                               images[1], images[2], images[3] if images[3] is not None else images[0])
         ctx.desc, ctx.t_stride, ctx.has4 = desc, int(t_stride), images[3] is not None and want_latent
@@ -814,7 +794,7 @@ class FieldTrainFunction(torch.autograd.Function):
                      ctx.t_stride, n, ptr(i1), ptr(i2), ptr(i3), ptr(i4) if ctx.has4 else None, ptr(table_f16),
                      ctypes.byref(ctx.desc), ptr(sigma), ptr(rgb), ptr(selector), ptr(saved), ptr(d_sigma), ptr(d_rgb),
                      ptr(dl), ptr(work), ptr(g1), ptr(g2), ptr(g3), ptr(g4) if dl is not None else None, ptr(gt), phase,
-                     ptr(ctx.order), ptr(ctx.n_dev), stream())
+                     ptr(ctx.n_dev), stream())
             if phase == 1:
                 hook(gt)  # the 191 MB table gradient is complete: its all-reduce overlaps the rest of the backward
-        return (g1, g2, g3, g4 if dl is not None else None, gt) + (None,) * 13
+        return (g1, g2, g3, g4 if dl is not None else None, gt) + (None,) * 12

@@ -79,7 +79,7 @@ class FieldOccEval:
         return self.field.query_density(x, self.rand_t(x.shape[0], x.device))["density"] * self.step
 
 
-def _field_fns(field, rays, timestamps, order_box=None):
+def _field_fns(field, rays, timestamps):
     def positions_of(t0, t1, ridx):
         o, d = rays.origins[ridx], rays.viewdirs[ridx]
         x = o + d * (t0 + t1)[:, None] / 2.0
@@ -109,7 +109,7 @@ def _field_fns(field, rays, timestamps, order_box=None):
                 and getattr(field, "fused_train_supported", lambda: False)()
                 and (timestamps.numel() == 1 or timestamps.numel() == rays.origins.shape[0])):
             return field.fused_train(ridx, t0, t1, rays.origins, rays.viewdirs, timestamps,
-                                     1 if timestamps.numel() == rays.origins.shape[0] else 0, order_box=order_box)
+                                     1 if timestamps.numel() == rays.origins.shape[0] else 0)
         if can_fuse(t0) and not field.training:
             sigma, rgb = fused(t0, t1, ridx, False)
             return rgb, {"density": sigma[:, None]}
@@ -137,9 +137,7 @@ def render_image(radiance_field, estimator, rays, near_plane=0.0, far_plane=1e10
     for i in range(0, n, chunk):
         cr = Rays(rays.origins[i:i + chunk], rays.viewdirs[i:i + chunk])
         ts = timestamps[i:i + chunk] if (radiance_field.training and timestamps is not None) else timestamps
-        # the estimator's region of interest (level 0) bounds the spatial buckets the training kernels walk the samples in
-        roi = estimator.aabbs_on_host()[0] if hasattr(estimator, "aabbs_on_host") else None
-        sigma_fn, rgb_sigma_fn = _field_fns(radiance_field, cr, ts, order_box=roi)
+        sigma_fn, rgb_sigma_fn = _field_fns(radiance_field, cr, ts)
         ridx, t0, t1 = estimator.sampling(cr.origins, cr.viewdirs, sigma_fn=sigma_fn, near_plane=near_plane,
                                           far_plane=far_plane, render_step_size=render_step_size,
                                           stratified=radiance_field.training, cone_angle=cone_angle,

@@ -210,7 +210,6 @@ int cednerf_field_train_fwd(const int64_t* ray_indices, const float* t_starts, c
                             const void* image_deform, const void* image_density, const void* image_colour,
                             const void* image_predict, const void* table_f16, const CednerfFieldDesc* desc, float* sigma,
                             float* rgb, float* latent, uint8_t* selector, float* move, void* saved,
-                            const int32_t* sample_order /*nullable: cednerf_sample_order*/,
                             const int64_t* n_device /*nullable: live sample count on the device, n = capacity*/,
                             void* stream);
 int cednerf_field_train_bwd(const int64_t* ray_indices, const float* t_starts, const float* t_ends, const float* rays_o,
@@ -221,20 +220,9 @@ int cednerf_field_train_bwd(const int64_t* ray_indices, const float* t_starts, c
                             const float* d_sigma, const float* d_rgb, const float* d_latent, void* work,
                             float* d_params_deform, float* d_params_density, float* d_params_colour,
                             float* d_params_predict, float* g_table, int phase,
-                            const int32_t* sample_order /*nullable, the forward's*/,
                             const int64_t* n_device /*nullable, as in the forward*/, void* stream);
 /* phase: 0 = the whole backward; 1 = colour and density nets + table gradient (g_table is complete on return: a
  * data-parallel caller starts its all-reduce here); 2 = the rest (predictor net, dL/dx of the encoding, deformation net). */
-
-/* Spatial bucket order of packed samples for the two calls above (csrc/sample_order.cu): `order` [n] int32 walks the live
- * samples bucket by bucket of a 128^3 Morton grid over the box [lo, hi] (position = o + d (t0 + t1) / 2), so that the
- * lanes of a warp are neighbours in space and the hash-grid gathers of the coarse and middle levels coalesce.  With an
- * order, kernel-internal sample s reads / writes entry order[s] of every per-sample array named in the signatures above;
- * `saved` and `work` are laid out by s.  workspace: cednerf_sample_order_workspace_bytes(n).  n_device nullable. */
-int64_t cednerf_sample_order_workspace_bytes(int64_t n);
-int cednerf_sample_order(const int64_t* ray_indices, const float* t_starts, const float* t_ends, const float* rays_o,
-                         const float* rays_d, int64_t n, const int64_t* n_device, float lo0, float lo1, float lo2,
-                         float hi0, float hi1, float hi2, void* workspace, int32_t* order, void* stream);
 
 /* ---- K4: compositing ------------------------------------------------------------------------------- */
 /* offsets[r] = first sample of ray r (ray_indices sorted); offsets[n_rays] = n_samples */

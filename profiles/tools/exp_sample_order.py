@@ -6,7 +6,7 @@ by a Morton key of their position - same samples, same results up to the permuta
 import sys, torch
 sys.path.insert(0, '/root/repo')
 import cednerf_b200 as cb
-from cednerf_b200 import workload as w, _lib, ops
+from cednerf_b200 import workload as w, _lib
 import bench
 DEV = torch.device('cuda:0')
 bits = int(sys.argv[1]) if len(sys.argv) > 1 else 7
@@ -28,14 +28,12 @@ def spread(v):
 key = spread(q[:, 0]) | (spread(q[:, 1]) << 1) | (spread(q[:, 2]) << 2)
 perm = torch.argsort(key)
 gs, gr = torch.randn(n, device=DEV) * 1e-3, torch.randn(n, 3, device=DEV) * 1e-3
-def run(order, label, product_order=False):
-    ops.SAMPLE_ORDER_MIN = 1 if product_order else None
+def run(order, label):
     ri, a0, a1 = (ridx[order], t0[order], t1[order]) if order is not None else (ridx, t0, t1)
     g0, g1 = (gs[order], gr[order]) if order is not None else (gs, gr)
     def step():
         for p in field.parameters(): p.grad = None
-        rgb, out = field.fused_train(ri, a0, a1, b['origins'], b['viewdirs'], b['timestamps'], 1,
-                                     order_box=cfg.roi_aabb if product_order else None)
+        rgb, out = field.fused_train(ri, a0, a1, b['origins'], b['viewdirs'], b['timestamps'], 1)
         lat = out['interal_output']['latent_losses']
         ((out['density'][:, 0] * g0).sum() + (rgb * g1).sum() + lat.mean()).backward()
         return rgb
@@ -51,9 +49,6 @@ def run(order, label, product_order=False):
     return rgb, [p.grad.clone() for p in field.parameters() if p.grad is not None]
 r0, g_ray = run(None, f'{n} samples, ray order    ')
 r1, g_sorted = run(perm, f'sorted by {3 * bits}-bit Morton key')
-r3, g_prod = run(None, 'ray order + cednerf_sample_order', product_order=True)
-print('product path: max |rgb diff|', float((r3 - r0).detach().abs().max()),
-      'gradient rel diff', [float((a - c).norm() / (c.norm() + 1e-30)) for a, c in zip(g_prod, g_ray)])
 # (c) whole RAYS reordered (samples stay packed per ray): key of a ray = Morton code of its point at the depth of the scene
 depth = float((lo + hi).norm()) * 0 + 1.6
 pr = b['origins'] + b['viewdirs'] * depth

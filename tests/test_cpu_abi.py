@@ -26,7 +26,7 @@ def test_library_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in the header but not exported"
     assert sorted(names) == _lib.exported_symbols()
-    assert lib.cednerf_abi_version() == 3
+    assert lib.cednerf_abi_version() == 4
 
 
 def test_ctypes_signatures_match_header():

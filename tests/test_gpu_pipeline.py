@@ -429,87 +429,3 @@ def test_interleaved_frames_match_frame_by_frame_rendering(cb):
     cb.render_images_test(1024, field, est, rays, ts, concurrency=2, render_bkgd=bk,
                           on_frame=lambda idx, res: seen.append((idx, res[3])), **rk)
     assert sorted(seen) == [(k, want[k][3]) for k in range(5)]
-
-
-def test_spatial_bucket_order_changes_nothing_but_the_walk(cb):
-    """cednerf_sample_order + the `sample_order` indirection of the fused training kernels: the same batch walked in
-    spatial buckets gives bit-identical per-sample outputs (every sample is computed independently) and gradients equal up
-    to fp32 summation order; the order is a permutation, deterministic, and identity on the unused tail of a
-    capacity-sized array.  Both the host-count and the device-count (capacity) paths."""
-    from cednerf_b200 import workload as w, ops
-
-    cfg = w.TINY
-    rk = w.render_kwargs(cfg)
-    est, field = w.build_scene(cfg, DEV, cb, seed=42)
-    est.train(), field.train()
-    b = {k: v.to(DEV) for k, v in w.draw_batch(cfg, 70000, torch.Generator().manual_seed(5)).items()}
-    rays = cb.Rays(b["origins"], b["viewdirs"])
-
-    def run(order_min, device_counts):
-        old, ops.SAMPLE_ORDER_MIN = ops.SAMPLE_ORDER_MIN, order_min
-        try:
-            for p in field.parameters():
-                p.grad = None
-            rgb, acc, depth, n_s, extra = cb.render_image(field, est, rays, render_bkgd=b["color_bkgd"],
-                                                          timestamps=b["timestamps"], jitter=b["jitter"],
-                                                          device_counts=device_counts, **rk)
-            loss = cb.losses.training_loss(rgb, acc, b["pixels"], extra, acc_entropy_loss=True, weight_rgbper=True,
-                                           use_feat_predict=True)
-            (loss * 1024.0).backward()
-            grads = {k: p.grad.detach().clone() for k, p in field.named_parameters() if p.grad is not None}
-            return rgb.detach(), extra[0], int(n_s), float(loss), grads
-        finally:
-            ops.SAMPLE_ORDER_MIN = old
-
-    plain = run(None, False)
-    n = plain[2]
-    assert n > 20000
-    for dc in (False, True, True):   # the first device-count call seeds the capacities through the host-count path
-        got = run(1, dc)
-        assert got[2] == n and torch.equal(got[0], plain[0])
-        for k in ("rgbs", "sigmas", "weights", "latent_losses"):
-            if k in plain[1] and torch.is_tensor(plain[1][k]):
-                assert torch.equal(got[1][k][:n] if got[1][k].shape[0] >= n and k != "latent_losses" else got[1][k],
-                                   plain[1][k]), k
-        assert abs(got[3] - plain[3]) <= 1e-6 * abs(plain[3])
-        for k, g in plain[4].items():
-            assert rel(got[4][k], g) <= 1e-5, (k, rel(got[4][k], g))
-    again = run(1, True)
-    for k, g in got[4].items():      # deterministic: the walk is a pure function of the inputs
-        assert rel(again[4][k], g) <= 2e-6, (k, rel(again[4][k], g))
-
-    # the order itself
-    ex = plain[1]
-    ridx, t0, t1 = ex["ray_indices"], ex["t_starts"], ex["t_ends"]
-    cap = n + 1000
-    ridx_p, t0_p, t1_p = (torch.cat([t, t.new_zeros(cap - n)]) for t in (ridx, t0, t1))   # bound: they outlive the launches
-    o_c, d_c = rays.origins.contiguous(), rays.viewdirs.contiguous()
-    n_dev = torch.tensor([n], dtype=torch.int64, device=DEV)
-    lib = cb._lib.load()
-    orders = []
-    for _ in range(2):
-        order = torch.full((cap,), -1, dtype=torch.int32, device=DEV)
-        ws = torch.empty(int(lib.cednerf_sample_order_workspace_bytes(cap)), dtype=torch.uint8, device=DEV)
-        cb._lib.call("cednerf_sample_order", cb._lib.ptr(ridx_p), cb._lib.ptr(t0_p), cb._lib.ptr(t1_p),
-                     cb._lib.ptr(o_c), cb._lib.ptr(d_c), cap, cb._lib.ptr(n_dev),
-                     -1.0, -1.0, -1.0, 1.0, 1.0, 1.0, cb._lib.ptr(ws), cb._lib.ptr(order), cb._lib.stream())
-        orders.append(order.cpu().long())
-    o = orders[0]
-    assert torch.equal(orders[0], orders[1])
-    assert torch.equal(torch.sort(o[:n])[0], torch.arange(n)) and torch.equal(o[n:], torch.arange(n, cap))
-    x = (rays.origins[ridx] + rays.viewdirs[ridx] * ((t0 + t1) / 2)[:, None]).cpu()
-    q = ((x + 1.0) / 2.0 * 128).clamp(0, 127).long()
-
-    def spread(v):
-        out = torch.zeros_like(v)
-        for i in range(7):
-            out |= ((v >> i) & 1) << (3 * i)
-        return out
-
-    key = spread(q[:, 0]) | (spread(q[:, 1]) << 1) | (spread(q[:, 2]) << 2)
-    walked = key[o[:n]]
-    # samples on a bucket boundary may fall either side (the kernel multiplies by 128 / extent, this check divides): the
-    # walk is sorted by key except for such samples
-    assert float((walked[1:] < walked[:-1]).float().mean()) < 1e-3
-    same = walked[1:] == walked[:-1]
-    assert bool((o[:n][1:][same] > o[:n][:-1][same]).all())      # ascending sample index inside a bucket
