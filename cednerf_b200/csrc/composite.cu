@@ -7,6 +7,8 @@
 // Samples are packed by ray (ray_indices sorted, as the marcher emits them); a group of G lanes
 // (G = 4..32, picked from the mean samples/ray) owns one ray and walks its samples in chunks of G with
 // shuffle scans: one forward exclusive scan of sigma*dt, one reverse exclusive scan in the backward.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace {
@@ -46,6 +48,38 @@ __device__ __forceinline__ float group_sum(float v, unsigned gm) {
 #pragma unroll
   for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(gm, v, o, G);
   return v;
+}
+
+// G from the mean samples per ray S / n_rays: <= 6 -> 4, <= 12 -> 8, <= 24 -> 16, else 32 (compared in integers)
+__host__ __device__ __forceinline__ int pick_group(int64_t S, int64_t n_rays) {
+  if (S <= 6 * n_rays) return 4;
+  if (S <= 12 * n_rays) return 8;
+  if (S <= 24 * n_rays) return 16;
+  return 32;
+}
+
+// The group width changes the order of the per-ray scans and sums, so it is part of the result.  The per-ray kernels take
+// it from the LIVE sample count offsets[n_rays] on the device (g_fixed = 0): a capacity-sized sample set (buffers larger
+// than the live prefix, ops.counts_of) then gives the same bits as the exact-size set, whatever its capacity.  The launch
+// is sized from the host's estimate and every group walks its rays in a grid-stride loop, so any G is covered.
+// f(std::integral_constant<int, G>{}, ray, gl, gm) runs once per ray on its G lanes; `return` in f moves to the next ray.
+template <int G, class F>
+__device__ __forceinline__ void ray_groups_g(int64_t n_rays, F& f) {
+  const int gl = threadIdx.x % G;
+  const unsigned gm = group_mask<G>();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x / G;
+  for (int64_t ray = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G; ray < n_rays; ray += stride)
+    f(std::integral_constant<int, G>{}, ray, gl, gm);
+}
+
+template <class F>
+__device__ __forceinline__ void for_each_ray_group(const int64_t* offsets, int64_t n_rays, int g_fixed, F f) {
+  switch (g_fixed > 0 ? g_fixed : pick_group(offsets[n_rays], n_rays)) {
+    case 4: ray_groups_g<4>(n_rays, f); break;
+    case 8: ray_groups_g<8>(n_rays, f); break;
+    case 16: ray_groups_g<16>(n_rays, f); break;
+    default: ray_groups_g<32>(n_rays, f); break;
+  }
 }
 
 // offsets[r] = index of the first sample whose ray index is >= r; offsets[n_rays] = S.
@@ -88,93 +122,92 @@ struct CompositeFwdArgs {
   int32_t* next_flags;
 };
 
-template <int G>
-__global__ void __launch_bounds__(256) composite_fwd_kernel(CompositeFwdArgs a) {
-  const int gl = threadIdx.x % G;
-  const unsigned gm = group_mask<G>();
-  const int64_t slot = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
-  bool live = slot < a.n_rays;
-  if (a.round_state && live && slot >= (int64_t)a.round_state[0]) live = false;
-  if (!a.next_flags && !live) return;  // whole groups exit together
-  const int64_t ray = live ? (a.slot_ray ? (int64_t)a.slot_ray[slot] : slot) : 0;
-  const int64_t s0 = live ? a.offsets[slot] : 0, s1 = live ? a.offsets[slot + 1] : 0;
-  float carry = 0.f, cr = 0.f, cg = 0.f, cb = 0.f, co = 0.f, cd = 0.f;
-  // mode 2: continue a ray across marching rounds - the transmittance so far is 1 - opacity[ray] (utils.py:274-281)
-  const float ray_prefix = (a.accumulate_inplace == 2 && s0 < s1) ? 1.f - a.opacity[ray] : 1.f;
-  for (int64_t base = s0; base < s1; base += G) {
-    const int64_t i = base + gl;
-    const bool ok = i < s1;
-    float ta = 0.f, tb = 0.f, sg = 0.f, pf = ray_prefix;
-    if (ok) {
-      ta = a.t0[i];
-      tb = a.t1[i];
-      sg = a.sigma[i];
-      if (a.prefix) pf = a.prefix[i];
-    }
-    const float sd = sg * (tb - ta);
-    const float incl = group_incl_scan<G>(sd, gl, gm);
-    const float T = expf(-(carry + (incl - sd))) * pf;
-    const float al = 1.f - expf(-sd);
-    const float w = T * al;
-    carry += __shfl_sync(gm, incl, G - 1, G);
-    if (ok) {
-      if (a.w) a.w[i] = w;
-      if (a.trans) a.trans[i] = T;
-      if (a.alpha) a.alpha[i] = al;
-      co += w;
-      cd += w * ((ta + tb) * 0.5f);
-      if (a.rgb) {
-        cr += w * a.rgb[3 * i];
-        cg += w * a.rgb[3 * i + 1];
-        cb += w * a.rgb[3 * i + 2];
+__global__ void __launch_bounds__(256, 8) composite_fwd_kernel(CompositeFwdArgs a, int g_fixed) {
+  for_each_ray_group(a.offsets, a.n_rays, g_fixed, [&](auto g_, int64_t slot, int gl, unsigned gm) {
+    constexpr int G = decltype(g_)::value;
+    bool live = true;
+    if (a.round_state && slot >= (int64_t)a.round_state[0]) live = false;
+    if (!a.next_flags && !live) return;  // whole groups exit together
+    const int64_t ray = live ? (a.slot_ray ? (int64_t)a.slot_ray[slot] : slot) : 0;
+    const int64_t s0 = live ? a.offsets[slot] : 0, s1 = live ? a.offsets[slot + 1] : 0;
+    float carry = 0.f, cr = 0.f, cg = 0.f, cb = 0.f, co = 0.f, cd = 0.f;
+    // mode 2: continue a ray across marching rounds - the transmittance so far is 1 - opacity[ray] (utils.py:274-281)
+    const float ray_prefix = (a.accumulate_inplace == 2 && s0 < s1) ? 1.f - a.opacity[ray] : 1.f;
+    for (int64_t base = s0; base < s1; base += G) {
+      const int64_t i = base + gl;
+      const bool ok = i < s1;
+      float ta = 0.f, tb = 0.f, sg = 0.f, pf = ray_prefix;
+      if (ok) {
+        ta = a.t0[i];
+        tb = a.t1[i];
+        sg = a.sigma[i];
+        if (a.prefix) pf = a.prefix[i];
       }
-    }
-  }
-  if (!a.opacity && !a.colors && !a.depth) return;
-  cr = group_sum<G>(cr, gm);
-  cg = group_sum<G>(cg, gm);
-  cb = group_sum<G>(cb, gm);
-  co = group_sum<G>(co, gm);
-  cd = group_sum<G>(cd, gm);
-  bool keep = false;  // round mode: this lane speaks for a ray that stays alive
-  if (gl == 0 && live) {
-    if (a.accumulate_inplace) {
-      if (a.colors) {
-        a.colors[3 * ray] += cr;
-        a.colors[3 * ray + 1] += cg;
-        a.colors[3 * ray + 2] += cb;
-      }
-      float op = co;
-      if (a.opacity) {
-        op += a.opacity[ray];
-        a.opacity[ray] = op;
-      }
-      if (a.depth) a.depth[ray] += cd;
-      // alive = (opacity <= 1 - early_stop_eps) & (n_samples == k)   (cednerf/utils.py:300-304)
-      if (a.next_flags) keep = op <= 1.f - a.alive_eps && a.slot_counts[slot] == a.round_state[1];
-    } else {
-      if (a.depth_raw) a.depth_raw[ray] = cd;
-      if (a.opacity) a.opacity[ray] = co;
-      if (a.depth) a.depth[ray] = cd / fmaxf(co, a.depth_eps);
-      if (a.colors) {
-        float br = 0.f, bg = 0.f, bb = 0.f;
-        if (a.bkgd) {
-          const float* b = a.bkgd + (int64_t)a.bkgd_stride * ray;
-          br = b[0] * (1.f - co);
-          bg = b[1] * (1.f - co);
-          bb = b[2] * (1.f - co);
+      const float sd = sg * (tb - ta);
+      const float incl = group_incl_scan<G>(sd, gl, gm);
+      const float T = expf(-(carry + (incl - sd))) * pf;
+      const float al = 1.f - expf(-sd);
+      const float w = T * al;
+      carry += __shfl_sync(gm, incl, G - 1, G);
+      if (ok) {
+        if (a.w) a.w[i] = w;
+        if (a.trans) a.trans[i] = T;
+        if (a.alpha) a.alpha[i] = al;
+        co += w;
+        cd += w * ((ta + tb) * 0.5f);
+        if (a.rgb) {
+          cr += w * a.rgb[3 * i];
+          cg += w * a.rgb[3 * i + 1];
+          cb += w * a.rgb[3 * i + 2];
         }
-        a.colors[3 * ray] = cr + br;
-        a.colors[3 * ray + 1] = cg + bg;
-        a.colors[3 * ray + 2] = cb + bb;
       }
     }
-  }
-  // round mode: a flag per slot (0 beyond the live part of the list); the next round's list is the ORDERED compaction
-  // of the flagged rays (scan + cednerf_render_round_compact), so the list stays in pixel order and the lanes of a warp
-  // keep marching neighbouring rays.  (Measured: an unordered per-ray atomic append cost 45 % in the marcher and 30 % in
-  // the field kernel; CTA-sized ordered chunks in arbitrary order still 12 % and 6 %.)
-  if (a.next_flags && gl == 0 && slot < a.n_rays) a.next_flags[slot] = keep ? 1 : 0;
+    if (!a.opacity && !a.colors && !a.depth) return;
+    cr = group_sum<G>(cr, gm);
+    cg = group_sum<G>(cg, gm);
+    cb = group_sum<G>(cb, gm);
+    co = group_sum<G>(co, gm);
+    cd = group_sum<G>(cd, gm);
+    bool keep = false;  // round mode: this lane speaks for a ray that stays alive
+    if (gl == 0 && live) {
+      if (a.accumulate_inplace) {
+        if (a.colors) {
+          a.colors[3 * ray] += cr;
+          a.colors[3 * ray + 1] += cg;
+          a.colors[3 * ray + 2] += cb;
+        }
+        float op = co;
+        if (a.opacity) {
+          op += a.opacity[ray];
+          a.opacity[ray] = op;
+        }
+        if (a.depth) a.depth[ray] += cd;
+        // alive = (opacity <= 1 - early_stop_eps) & (n_samples == k)   (cednerf/utils.py:300-304)
+        if (a.next_flags) keep = op <= 1.f - a.alive_eps && a.slot_counts[slot] == a.round_state[1];
+      } else {
+        if (a.depth_raw) a.depth_raw[ray] = cd;
+        if (a.opacity) a.opacity[ray] = co;
+        if (a.depth) a.depth[ray] = cd / fmaxf(co, a.depth_eps);
+        if (a.colors) {
+          float br = 0.f, bg = 0.f, bb = 0.f;
+          if (a.bkgd) {
+            const float* b = a.bkgd + (int64_t)a.bkgd_stride * ray;
+            br = b[0] * (1.f - co);
+            bg = b[1] * (1.f - co);
+            bb = b[2] * (1.f - co);
+          }
+          a.colors[3 * ray] = cr + br;
+          a.colors[3 * ray + 1] = cg + bg;
+          a.colors[3 * ray + 2] = cb + bb;
+        }
+      }
+    }
+    // round mode: a flag per slot (0 beyond the live part of the list); the next round's list is the ORDERED compaction
+    // of the flagged rays (scan + cednerf_render_round_compact), so the list stays in pixel order and the lanes of a warp
+    // keep marching neighbouring rays.  (Measured: an unordered per-ray atomic append cost 45 % in the marcher and 30 % in
+    // the field kernel; CTA-sized ordered chunks in arbitrary order still 12 % and 6 %.)
+    if (a.next_flags && gl == 0) a.next_flags[slot] = keep ? 1 : 0;
+  });
 }
 
 struct CompositeBwdArgs {
@@ -200,99 +233,95 @@ struct CompositeBwdArgs {
   float depth_eps;
 };
 
-template <int G>
 __global__ void __launch_bounds__(256) composite_bwd_kernel(CompositeBwdArgs a) {
-  const int gl = threadIdx.x % G;
-  const unsigned gm = group_mask<G>();
-  const int64_t ray = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
-  if (ray >= a.n_rays) return;
-  const int64_t s0 = a.offsets[ray], s1 = a.offsets[ray + 1];
-  if (s0 >= s1) return;
-  // per-ray upstream gradients, folded back through depth normalisation and background blend
-  float gcr = 0.f, gcg = 0.f, gcb = 0.f, gO = 0.f, gD = 0.f;
-  if (a.g_colors) {
-    gcr = a.g_colors[3 * ray];
-    gcg = a.g_colors[3 * ray + 1];
-    gcb = a.g_colors[3 * ray + 2];
-    if (a.bkgd) {
-      const float* b = a.bkgd + (int64_t)a.bkgd_stride * ray;
-      gO -= gcr * b[0] + gcg * b[1] + gcb * b[2];
-    }
-  }
-  if (a.g_opacity) gO += a.g_opacity[ray];
-  if (a.g_depth && a.opacity && a.depth_raw) {
-    const float o = a.opacity[ray], gd = a.g_depth[ray];
-    const float den = fmaxf(o, a.depth_eps);
-    gD = gd / den;
-    if (o > a.depth_eps) gO -= gd * a.depth_raw[ray] / (den * den);
-  }
-  float carry = 0.f;  // sum over later samples of GT_s * T_s
-  const int64_t n = s1 - s0;
-  const int64_t n_chunks = (n + G - 1) / G;
-  for (int64_t c = n_chunks - 1; c >= 0; --c) {
-    const int64_t i = s0 + c * G + gl;
-    const bool ok = i < s1;
-    float T = 0.f, al = 0.f, ta = 0.f, tb = 0.f, r = 0.f, g = 0.f, b = 0.f;
-    float gw = 0.f, gT = 0.f, ga = 0.f;
-    if (ok) {
-      T = a.trans[i];
-      al = a.alpha[i];
-      ta = a.t0[i];
-      tb = a.t1[i];
-      if (a.rgb) {
-        r = a.rgb[3 * i];
-        g = a.rgb[3 * i + 1];
-        b = a.rgb[3 * i + 2];
-      }
-      if (a.g_w) gw = a.g_w[i];
-      if (a.g_trans) gT = a.g_trans[i];
-      if (a.g_alpha) ga = a.g_alpha[i];
-    }
-    gw += gcr * r + gcg * g + gcb * b + gO + gD * ((ta + tb) * 0.5f);
-    const float GT = gT + gw * al;
-    const float GA = ga + gw * T;
-    const float v = ok ? GT * T : 0.f;
-    const float incl = group_incl_scan_rev<G>(v, gl, gm);
-    const float later = carry + (incl - v);
-    carry += __shfl_sync(gm, incl, 0, G);
-    if (ok) {
-      a.g_sigma[i] = (tb - ta) * (GA * (1.f - al) - later);
-      if (a.g_rgb) {
-        const float w = T * al;
-        a.g_rgb[3 * i] = w * gcr;
-        a.g_rgb[3 * i + 1] = w * gcg;
-        a.g_rgb[3 * i + 2] = w * gcb;
+  for_each_ray_group(a.offsets, a.n_rays, 0, [&](auto g_, int64_t ray, int gl, unsigned gm) {
+    constexpr int G = decltype(g_)::value;
+    const int64_t s0 = a.offsets[ray], s1 = a.offsets[ray + 1];
+    if (s0 >= s1) return;
+    // per-ray upstream gradients, folded back through depth normalisation and background blend
+    float gcr = 0.f, gcg = 0.f, gcb = 0.f, gO = 0.f, gD = 0.f;
+    if (a.g_colors) {
+      gcr = a.g_colors[3 * ray];
+      gcg = a.g_colors[3 * ray + 1];
+      gcb = a.g_colors[3 * ray + 2];
+      if (a.bkgd) {
+        const float* b = a.bkgd + (int64_t)a.bkgd_stride * ray;
+        gO -= gcr * b[0] + gcg * b[1] + gcb * b[2];
       }
     }
-  }
+    if (a.g_opacity) gO += a.g_opacity[ray];
+    if (a.g_depth && a.opacity && a.depth_raw) {
+      const float o = a.opacity[ray], gd = a.g_depth[ray];
+      const float den = fmaxf(o, a.depth_eps);
+      gD = gd / den;
+      if (o > a.depth_eps) gO -= gd * a.depth_raw[ray] / (den * den);
+    }
+    float carry = 0.f;  // sum over later samples of GT_s * T_s
+    const int64_t n = s1 - s0;
+    const int64_t n_chunks = (n + G - 1) / G;
+    for (int64_t c = n_chunks - 1; c >= 0; --c) {
+      const int64_t i = s0 + c * G + gl;
+      const bool ok = i < s1;
+      float T = 0.f, al = 0.f, ta = 0.f, tb = 0.f, r = 0.f, g = 0.f, b = 0.f;
+      float gw = 0.f, gT = 0.f, ga = 0.f;
+      if (ok) {
+        T = a.trans[i];
+        al = a.alpha[i];
+        ta = a.t0[i];
+        tb = a.t1[i];
+        if (a.rgb) {
+          r = a.rgb[3 * i];
+          g = a.rgb[3 * i + 1];
+          b = a.rgb[3 * i + 2];
+        }
+        if (a.g_w) gw = a.g_w[i];
+        if (a.g_trans) gT = a.g_trans[i];
+        if (a.g_alpha) ga = a.g_alpha[i];
+      }
+      gw += gcr * r + gcg * g + gcb * b + gO + gD * ((ta + tb) * 0.5f);
+      const float GT = gT + gw * al;
+      const float GA = ga + gw * T;
+      const float v = ok ? GT * T : 0.f;
+      const float incl = group_incl_scan_rev<G>(v, gl, gm);
+      const float later = carry + (incl - v);
+      carry += __shfl_sync(gm, incl, 0, G);
+      if (ok) {
+        a.g_sigma[i] = (tb - ta) * (GA * (1.f - al) - later);
+        if (a.g_rgb) {
+          const float w = T * al;
+          a.g_rgb[3 * i] = w * gcr;
+          a.g_rgb[3 * i + 1] = w * gcg;
+          a.g_rgb[3 * i + 2] = w * gcb;
+        }
+      }
+    }
+  });
 }
 
 // visibility mask of nerfacc's render_visibility_from_density, fused with the scan
-template <int G>
 __global__ void __launch_bounds__(256)
 visibility_kernel(const float* __restrict__ t0, const float* __restrict__ t1, const float* __restrict__ sigma,
                   const int64_t* __restrict__ offsets, int64_t n_rays, float early_stop_eps, float alpha_thre,
                   uint8_t* __restrict__ keep, int32_t* __restrict__ kept_counts) {
-  const int gl = threadIdx.x % G;
-  const unsigned gm = group_mask<G>();
-  const int64_t ray = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
-  if (ray >= n_rays) return;
-  const int64_t s0 = offsets[ray], s1 = offsets[ray + 1];
-  float carry = 0.f;
-  int kept = 0;
-  for (int64_t base = s0; base < s1; base += G) {
-    const int64_t i = base + gl;
-    const bool ok = i < s1;
-    const float sd = ok ? sigma[i] * (t1[i] - t0[i]) : 0.f;
-    const float incl = group_incl_scan<G>(sd, gl, gm);
-    const float T = expf(-(carry + (incl - sd)));
-    const float al = 1.f - expf(-sd);
-    carry += __shfl_sync(gm, incl, G - 1, G);
-    const bool k = ok && (T >= early_stop_eps) && (alpha_thre <= 0.f || al >= alpha_thre);
-    if (ok) keep[i] = k;
-    if (kept_counts) kept += __popc(__ballot_sync(gm, k) & gm);
-  }
-  if (kept_counts && gl == 0) kept_counts[ray] = kept;
+  for_each_ray_group(offsets, n_rays, 0, [&](auto g_, int64_t ray, int gl, unsigned gm) {
+    constexpr int G = decltype(g_)::value;
+    const int64_t s0 = offsets[ray], s1 = offsets[ray + 1];
+    float carry = 0.f;
+    int kept = 0;
+    for (int64_t base = s0; base < s1; base += G) {
+      const int64_t i = base + gl;
+      const bool ok = i < s1;
+      const float sd = ok ? sigma[i] * (t1[i] - t0[i]) : 0.f;
+      const float incl = group_incl_scan<G>(sd, gl, gm);
+      const float T = expf(-(carry + (incl - sd)));
+      const float al = 1.f - expf(-sd);
+      carry += __shfl_sync(gm, incl, G - 1, G);
+      const bool k = ok && (T >= early_stop_eps) && (alpha_thre <= 0.f || al >= alpha_thre);
+      if (ok) keep[i] = k;
+      if (kept_counts) kept += __popc(__ballot_sync(gm, k) & gm);
+    }
+    if (kept_counts && gl == 0) kept_counts[ray] = kept;
+  });
 }
 
 // Compaction of the visible samples (what OccGridEstimator.sampling returns): every ray's kept samples move, in order,
@@ -328,24 +357,22 @@ compact_samples_kernel(const uint8_t* __restrict__ keep, const int64_t* __restri
 }
 
 // generic per-ray weighted sum of C channels: out[r,c] (+)= sum_s w_s * v[s,c]   (v null -> 1)
-template <int G>
-__global__ void __launch_bounds__(256)
+__global__ void __launch_bounds__(256, 8)
 accumulate_fwd_kernel(const float* __restrict__ w, const float* __restrict__ v, int C,
                       const int64_t* __restrict__ offsets, int64_t n_rays, float* __restrict__ out, int inplace) {
-  const int gl = threadIdx.x % G;
-  const unsigned gm = group_mask<G>();
-  const int64_t ray = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
-  if (ray >= n_rays) return;
-  const int64_t s0 = offsets[ray], s1 = offsets[ray + 1];
-  for (int c = 0; c < C; ++c) {
-    float acc = 0.f;
-    for (int64_t i = s0 + gl; i < s1; i += G) acc += w[i] * (v ? v[i * C + c] : 1.f);
-    acc = group_sum<G>(acc, gm);
-    if (gl == 0) {
-      if (inplace) out[ray * C + c] += acc;
-      else out[ray * C + c] = acc;
+  for_each_ray_group(offsets, n_rays, 0, [&](auto g_, int64_t ray, int gl, unsigned gm) {
+    constexpr int G = decltype(g_)::value;
+    const int64_t s0 = offsets[ray], s1 = offsets[ray + 1];
+    for (int c = 0; c < C; ++c) {
+      float acc = 0.f;
+      for (int64_t i = s0 + gl; i < s1; i += G) acc += w[i] * (v ? v[i * C + c] : 1.f);
+      acc = group_sum<G>(acc, gm);
+      if (gl == 0) {
+        if (inplace) out[ray * C + c] += acc;
+        else out[ray * C + c] = acc;
+      }
     }
-  }
+  });
 }
 
 __global__ void accumulate_bwd_kernel(const float* __restrict__ w, const float* __restrict__ v, int C,
@@ -446,15 +473,11 @@ accumulate_c32_bwd_kernel(const float* __restrict__ w, const float4* __restrict_
   }
 }
 
-int pick_group(int64_t S, int64_t n_rays) {
-  const double mean = n_rays > 0 ? (double)S / (double)n_rays : 0.0;
-  if (mean <= 6.0) return 4;
-  if (mean <= 12.0) return 8;
-  if (mean <= 24.0) return 16;
-  return 32;
-}
-
 }  // namespace
+
+// kernels that choose their group width on the device: the grid has G lanes per ray for the host's estimate of G
+#define LAUNCH_PER_RAY(KERNEL, S_, ...)                                                                      \
+  KERNEL<<<cednerf_blocks(n_rays * pick_group(S_, n_rays), 256), 256, 0, st>>>(__VA_ARGS__)
 
 #define DISPATCH_G(G_, KERNEL, ...)                                                          \
   do {                                                                                       \
@@ -486,7 +509,7 @@ CEDNERF_EXPORT int cednerf_composite_fwd(const float* t_starts, const float* t_e
   cudaStream_t st = (cudaStream_t)stream;
   CompositeFwdArgs a{t_starts, t_ends, sigmas, rgbs, prefix_trans, offsets, bkgd, bkgd_stride, n_rays, weights,
                      trans, alphas, colors, opacity, depth, depth_raw, accumulate_inplace, depth_eps};
-  DISPATCH_G(pick_group(n_samples, n_rays), composite_fwd_kernel, a);
+  LAUNCH_PER_RAY(composite_fwd_kernel, n_samples, a, 0);
   return cednerf_check_launch("cednerf_composite_fwd");
 }
 
@@ -507,7 +530,9 @@ CEDNERF_EXPORT int cednerf_render_round_composite(const float* t_starts, const f
   CompositeFwdArgs a{t_starts, t_ends, sigmas, rgbs, nullptr, offsets, nullptr, 0, n_bound, nullptr, nullptr, nullptr,
                      colors, opacity, depth, nullptr, 2, 0.f, alive, round_state, slot_counts, early_stop_eps, alive_flags};
   const int64_t n_rays = n_bound;
-  DISPATCH_G(pick_group((int64_t)k_hint * n_bound, n_bound), composite_fwd_kernel, a);
+  // the group width of a round follows k_hint, not the live count: the rounds' launches are fixed in advance
+  const int g = pick_group((int64_t)k_hint * n_bound, n_bound);
+  composite_fwd_kernel<<<cednerf_blocks(n_rays * g, 256), 256, 0, st>>>(a, g);
   return cednerf_check_launch("cednerf_render_round_composite");
 }
 
@@ -551,7 +576,7 @@ CEDNERF_EXPORT int cednerf_composite_bwd(const float* t_starts, const float* t_e
   cudaStream_t st = (cudaStream_t)stream;
   CompositeBwdArgs a{t_starts, t_ends, rgbs, trans, alphas, offsets, bkgd, bkgd_stride, n_rays, opacity, depth_raw,
                      g_colors, g_opacity, g_depth, g_weights, g_trans, g_alphas, g_sigmas, g_rgbs, depth_eps};
-  DISPATCH_G(pick_group(n_samples, n_rays), composite_bwd_kernel, a);
+  LAUNCH_PER_RAY(composite_bwd_kernel, n_samples, a);
   return cednerf_check_launch("cednerf_composite_bwd");
 }
 
@@ -562,7 +587,7 @@ CEDNERF_EXPORT int cednerf_visibility_mask(const float* t_starts, const float* t
   CEDNERF_REQUIRE(n_rays >= 0 && n_samples >= 0, "bad sizes");
   if (n_rays == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  DISPATCH_G(pick_group(n_samples, n_rays), visibility_kernel, t_starts, t_ends, sigmas, offsets, n_rays,
+  LAUNCH_PER_RAY(visibility_kernel, n_samples, t_starts, t_ends, sigmas, offsets, n_rays,
              early_stop_eps, alpha_thre, keep, kept_counts);
   return cednerf_check_launch("cednerf_visibility_mask");
 }
@@ -611,7 +636,7 @@ CEDNERF_EXPORT int cednerf_accumulate_fwd(const float* weights, const float* val
                                                                                  n_rays, outputs, inplace);
     return cednerf_check_launch("cednerf_accumulate_fwd");
   }
-  DISPATCH_G(pick_group(n_samples, n_rays), accumulate_fwd_kernel, weights, values, n_channels, offsets, n_rays,
+  LAUNCH_PER_RAY(accumulate_fwd_kernel, n_samples, weights, values, n_channels, offsets, n_rays,
              outputs, inplace);
   return cednerf_check_launch("cednerf_accumulate_fwd");
 }

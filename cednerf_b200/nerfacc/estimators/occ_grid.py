@@ -91,28 +91,36 @@ class OccGridEstimator(torch.nn.Module):
     def _capacity(self, kind: str):
         st = self._cap_state.setdefault(kind, {"last": None, "pending": [], "ring": [], "next": 0})
         while st["pending"] and st["pending"][0][0].query():
-            _, host, cap = st["pending"].pop(0)
+            _, host, cap, marched = st["pending"].pop(0)
             raw = int(host[1])
             st["last"] = raw
             if raw > cap:
                 self.dropped_samples += raw - cap
+            if marched is not None and int(marched[1]) > int(marched[0]):
+                # the visible samples of a truncated marched set: scaled up to the whole set (and at most all of it),
+                # or the next batch would outgrow this capacity as well
+                kept_m, raw_m = int(marched[0]), int(marched[1])
+                st["last"] = min(-(-raw * raw_m // kept_m), raw_m) if kept_m else raw_m
         if st["last"] is None:
             return None
         return ops._sticky_capacity(max(int(st["last"] * self._HEADROOM), 65536))
 
-    def _note_totals(self, kind: str, totals: torch.Tensor, cap: int):
+    def _note_totals(self, kind: str, totals: torch.Tensor, cap: int, marched: Optional[torch.Tensor] = None):
+        """Queue the copy of a batch's totals (and, for the visible ones, the same batch's marched totals) to the host."""
         st = self._cap_state[kind]
         if not st["ring"]:
-            st["ring"] = [torch.empty(2, dtype=torch.int64).pin_memory() for _ in range(32)]
+            st["ring"] = [tuple(torch.empty(2, dtype=torch.int64).pin_memory() for _ in range(2)) for _ in range(32)]
         if len(st["pending"]) >= len(st["ring"]):   # the host ran 32 batches ahead of the device: wait for the oldest
             st["pending"][0][0].synchronize()
             self._capacity(kind)
-        host = st["ring"][st["next"] % len(st["ring"])]
+        host, host_m = st["ring"][st["next"] % len(st["ring"])]
         st["next"] += 1
         host.copy_(totals, non_blocking=True)
+        if marched is not None:
+            host_m.copy_(marched, non_blocking=True)
         ev = torch.cuda.Event()
         ev.record()
-        st["pending"].append((ev, host, cap))
+        st["pending"].append((ev, host, cap, None if marched is None else host_m))
 
     def _seed_capacity(self, kind: str, total: int):
         self._cap_state.setdefault(kind, {"last": None, "pending": [], "ring": [], "next": 0})["last"] = int(total)
@@ -142,7 +150,7 @@ class OccGridEstimator(torch.nn.Module):
         assert sigmas.shape == t0.shape, f"sigmas must have shape {tuple(t0.shape)}"
         k_idx, k_t0, k_t1, k_off, k_tot = ops.visible_samples_capped(t0, t1, sigmas, offsets, n, early_stop_eps,
                                                                      min(alpha_thre, self._occs_mean()), cap_v)
-        self._note_totals("visible", k_tot, cap_v)
+        self._note_totals("visible", k_tot, cap_v, totals)
         k_idx._cednerf_counts = (k_off, k_tot[0:1])
         return k_idx, k_t0, k_t1
 
